@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/sec of the AOT mask-propagation hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model r50_aotl]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model r50_aotl] [--dump-outputs DIR]
 
 One "step" = one propagated frame through the reference's timed span (networks/managers/
 evaluator.py:325-446): match_propogate_one_frame + decode + softmax/argmax + nearest resize +
@@ -9,6 +9,10 @@ update_memory; the reference frame is excluded, as in the reference.  Workload =
 configs[1]: R50-AOTL, synthetic 480p (481x849 network input, 480x854 output), 10 objects, long-term
 gap 5, fp32; K = 99 steps is exactly the 100-frame clip.  Warm-up runs W frames of a scratch clip,
 then the engine is restarted so the timed clip starts from an empty memory bank.
+
+--dump-outputs DIR writes what the timed value pass handed back at its last step K (rank 0), as float32 .npy:
+label.npy (the 480x854 label map) and logits.npy (the decoder's low-resolution logits of the background and the 10
+objects).  Weights and clip are seeded, so the same arguments give the same inputs on every run and build.
 
 Prints ONE JSON line (rank 0).  `value`: inputs resident in HBM, fused mask path.  `e2e`: the
 drop-in API exactly as the unedited evaluator drives it, with pinned HOST frames copied H2D and
@@ -118,14 +122,14 @@ def step_fused(eng, img):
     """value path: all-kernel span, label map produced by the fused upsample+argmax kernel."""
     from aot_benchmark_b200 import ops
     eng.match_propogate_one_frame(img)
-    eng.decode_current_logits(None)
+    logits = eng.decode_current_logits(None)
     e0 = eng.aot_engines[0]
     label = torch.empty((1, 1, H_OUT, W_OUT), dtype=torch.float32, device=img.device)
     ops.logits_argmax(e0.pred_id_logits, label, e0.align_corners)
     small = torch.empty((1, 1) + tuple(eng.input_size_2d), dtype=torch.float32, device=img.device)
     ops.nearest_resize(label, small)
     eng.update_memory(small)
-    return label
+    return label, logits
 
 
 def step_dropin(eng, img_host, label_host, stream_dev):
@@ -138,6 +142,14 @@ def step_dropin(eng, img_host, label_host, stream_dev):
     fb = F.interpolate(label, size=eng.input_size_2d, mode="nearest")
     eng.update_memory(fb)
     label_host.copy_(label.to(torch.uint8), non_blocking=True)   # the mask the evaluator writes out
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: {name: CPU float tensor} -> out_dir/<name>.npy"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 def run_ours(args):
@@ -163,10 +175,7 @@ def run_ours(args):
         if world < 2:
             raise SystemExit("--mode shard needs torchrun with >= 2 ranks (the bank is sharded over ranks)")
         eng.enable_kv_sharding(rank, world)
-    FULL = 99                                          # BASELINE configs[1]: 1 reference + 99 propagated frames
-    want_full = (K != FULL) and not args.no_full_clip and not shard
-    n_frames = (max(K, FULL) if want_full else K) + 1
-    frames, mask = make_clip(n_frames, seed=1234 + (0 if shard else rank))
+    frames, mask = make_clip(K + 1, seed=1234 + (0 if shard else rank))
     frames_dev = [f.to(dev) for f in frames]          # ~4.9 MB each, 490 MB for the clip: larger than L2
     frames_host = [f.pin_memory() for f in frames]
     mask_dev = mask.to(dev)
@@ -179,7 +188,8 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def run_clip(mode, n_steps):
+    def run_clip(mode, n_steps, keep=None):
+        """keep: a dict that receives, after the timed region, host copies of what the last fused step returned."""
         eng.restart_engine()
         with torch.no_grad():
             eng.add_reference_frame(frames_dev[0], mask_dev, obj_nums=[OBJS], frame_step=0)
@@ -189,12 +199,16 @@ def run_ours(args):
             ev0.record()
             for t in range(1, n_steps + 1):
                 if mode == "fused":
-                    step_fused(eng, frames_dev[t])
+                    res = step_fused(eng, frames_dev[t])
                 else:
                     step_dropin(eng, frames_host[t], label_host, dev)
             ev1.record()
             barrier()
             l1 = L.aotb_launch_count() + engine_mod.REPLAYED_KERNELS[0]
+            if keep is not None:
+                label, logits = res
+                keep["label"] = label[0, 0].float().cpu()
+                keep["logits"] = logits[0, :OBJS + 1].float().cpu()
         ms = ev0.elapsed_time(ev1)
         if dist is not None:
             t = torch.tensor([ms], device=dev)
@@ -211,13 +225,13 @@ def run_ours(args):
     peak = peaks.get("bf16_tflops_sustained", peaks["bf16_tflops"])
     clips = 1 if shard else world            # shard mode: one clip, total work fixed -> strong scaling
 
-    def measure(n_steps, sample_clocks):
+    def measure(n_steps, sample_clocks, keep=None):
         """value pass (fused mask path, resident inputs, CUDA graphs), e2e pass (drop-in API, pinned host frames), probe pass
         (same clip, eager launches, CUDA events around every long-term attention and every tensor-core conv launch)."""
         sampler = ClockSampler(local)
         if sample_clocks and rank == 0:
             sampler.start()
-        ms_value, launches = run_clip("fused", n_steps)
+        ms_value, launches = run_clip("fused", n_steps, keep)
         clocks = sampler.stop() if (sample_clocks and rank == 0) else None
         ms_e2e, _ = run_clip("dropin", n_steps)
         lt_probe, conv_probe = [], []
@@ -283,8 +297,8 @@ def run_ours(args):
                 "conv_launches": len(probe), "gflop": round(flops / 1e9, 2), "ms": round(ms, 4),
                 "achieved": round(ach, 2), "unit": "TFLOP/s", "frac": round(ach / peak, 4)}
 
-    m = measure(K, True)
-    m_full = measure(FULL, False) if want_full else None
+    last = {} if args.dump_outputs and rank == 0 else None
+    m = measure(K, True, last)
     enc = encoder_probe() if cfg.MODEL_ENCODER == "resnet50" else None
     enc_hw = eng.aot_engines[0].enc_hw
     h2d_bytes = int(frames_host[1].numel() * 4)
@@ -294,6 +308,8 @@ def run_ours(args):
         eng.restart_engine()
         torch.cuda.empty_cache()
         cfg4 = measure_cfg4(args.cfg4_frames, rank, world, dev, dist)
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     if rank != 0:
         if dist is not None:
             dist.destroy_process_group()
@@ -334,14 +350,6 @@ def run_ours(args):
         "roofline_conv": dict(conv_roofline(m, K), encoder=enc),
         "clocks": m["clocks"],
     }
-    if m_full is not None:
-        # the BASELINE configs[1] clip in full (the bank reaches 20 memory frames), whatever --steps the driver passed
-        fl = {"kernel": lt_name, "bound": "tensor"}
-        fl.update(lt_roofline(m_full, FULL))
-        out["full_clip"] = {"steps": FULL, "value": round(clips * FULL / (m_full["ms_value"] / 1e3), 3), "unit": "frames/s",
-                            "ms_per_step": round(m_full["ms_value"] / FULL, 4),
-                            "e2e": round(clips * FULL / (m_full["ms_e2e"] / 1e3), 3), "gpu_launches": m_full["launches"],
-                            "roofline": fl, "roofline_conv": conv_roofline(m_full, FULL)}
     if cfg4 is not None:
         out["cfg4"] = cfg4
     if not args.skip_cpu_baseline:
@@ -585,8 +593,8 @@ def main():
     ap.add_argument("--cfg4-frames", type=int, default=int(os.environ.get("AOTB_BENCH_CFG4_FRAMES", "500")),
                     help="propagated frames of the additional BASELINE configs[3] record (SwinB-AOTL, one clip, long-term bank "
                          "sharded over the GPUs when N > 1); 0 disables it")
-    ap.add_argument("--no-full-clip", action="store_true",
-                    help="development only: when --steps != 99, skip the additional 99-frame full_clip sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the label map and logits of the value pass's last timed step to DIR/<name>.npy (float32)")
     ap.add_argument("--skip-cpu-baseline", action="store_true",
                     help="development only: omit the cpu_baseline leg (the driver's default run keeps it)")
     args = ap.parse_args()

@@ -283,6 +283,39 @@ def io_case(out_dir):
     torch.save(out, os.path.join(out_dir, "io_side.pt"))
 
 
+CONTRACT_MODELS = ["aott", "r50_aotl", "deaott", "r50_deaotl", "swinb_aotl", "swinb_deaotl"]
+
+
+def contract_case(out_dir):
+    """What the tests check against the reference without importing it (tests/golden/reference_contract.json.gz): per model
+    the state_dict (key -> shape) and the repr of every config value, the DAVIS palette table, and the
+    layout of the reference's ``networks`` package with the ``from networks.* import`` statements of each module (the seam
+    the overlay package replaces)."""
+    import ast
+    import gzip
+    import json
+    import utils.image as RI
+    from aot_benchmark_b200 import EngineConfig, build_vos_model
+    out = {"models": {}, "palette": list(RI._palette), "networks": {}}
+    for m in CONTRACT_MODELS:
+        rc, mc = DefaultEngineConfig("x", m), EngineConfig("x", m)
+        out["models"][m] = {
+            "state_dict": {k: list(v.shape) for k, v in ref_build_model(rc.MODEL_VOS, rc).state_dict().items()},
+            "config": {k: repr(v) for k, v in rc.__dict__.items() if k not in ("EXP_NAME", "MODEL_NAME")}}
+        b = {k: list(v.shape) for k, v in build_vos_model(mc.MODEL_VOS, mc).state_dict().items()}
+        print(f"[contract {m}] {len(b)} parameters, state_dict matches the reference: {b == out['models'][m]['state_dict']}")
+    root = os.path.join(REF, "networks")
+    for d, _, files in sorted(os.walk(root)):
+        for f in sorted(files):
+            if f.endswith(".py"):
+                path = os.path.join(d, f)
+                imports = [[n.module, [a.name for a in n.names]] for n in ast.walk(ast.parse(open(path).read()))
+                           if isinstance(n, ast.ImportFrom) and n.module and n.module.split(".")[0] == "networks"]
+                out["networks"][os.path.relpath(path, REF)] = imports
+    with gzip.GzipFile(os.path.join(out_dir, "reference_contract.json.gz"), "wb", mtime=0) as fh:   # byte-reproducible
+        fh.write(json.dumps(out, sort_keys=True).encode())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=os.path.join(REPO, "tests", "golden"))
@@ -300,6 +333,8 @@ def main():
             events_case(a.out, name)
     if a.only == "io":
         io_case(a.out)
+    if a.only in (None, "contract"):
+        contract_case(a.out)
     for name in FULL_CASES:
         if a.only in ("full", name):              # not part of the default regeneration (minutes of CPU)
             full_case(name, a.out)

@@ -12,18 +12,14 @@ GOLDEN = os.path.join(REPO, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference checkout at /root/reference")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
     has_gpu = torch.cuda.is_available()
-    has_ref = os.path.isdir(os.environ.get("AOT_REFERENCE", "/root/reference"))
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="reference checkout not present (GPU box)"))
 
 
 @pytest.fixture(scope="session")

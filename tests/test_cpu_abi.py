@@ -11,6 +11,12 @@ import torch
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+def _cuobjdump(*args):
+    """cuobjdump of the toolkit whose nvcc built the library (found next to it, not on PATH)."""
+    from aot_benchmark_b200.build import NVCC
+    return subprocess.run([os.path.join(os.path.dirname(NVCC), "cuobjdump"), *args], capture_output=True, text=True)
+
+
 def test_library_exports_every_declared_symbol():
     from aot_benchmark_b200 import _lib
     decl = _lib.parse_header()
@@ -25,7 +31,7 @@ def test_library_exports_every_declared_symbol():
 
 def test_sass_is_sm100a_only():
     from aot_benchmark_b200 import _lib
-    r = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True)
+    r = _cuobjdump("-lelf", _lib.LIB_PATH)
     if r.returncode != 0:
         pytest.skip("cuobjdump unavailable")
     archs = {l.split(".")[-2] for l in r.stdout.splitlines() if "sm_" in l}
@@ -76,16 +82,21 @@ def test_separate_mask_matches_reference_semantics(monkeypatch):
     eng.aot_engines = []
 
 
-@pytest.mark.reference
-def test_overlay_resolves_in_front_of_reference():
-    code = ("import sys; sys.path[:0]=[%r, %r, '/root/reference'];"
+def test_overlay_resolves_in_front_of_reference(golden_dir, tmp_path):
+    """The overlay in front of a reference checkout (a stand-in with the reference's recorded `networks` layout and imports):
+    engines and models resolve to this package, everything else -- and the evaluator's own imports -- to the checkout."""
+    from oracle.fixtures import load_reference_contract, write_reference_standin
+    ref = str(tmp_path / "reference")
+    write_reference_standin(ref, load_reference_contract(golden_dir)["networks"])
+    code = ("import sys; sys.path[:0]=[%r, %r, %r];"
             "from networks.engines import build_engine; from networks.models import build_vos_model;"
-            "import networks.layers.attention as A; from networks.managers.evaluator import Evaluator;"
+            "import networks.layers.attention as A; import networks.managers.evaluator as E;"
             "assert build_engine.__module__=='aot_benchmark_b200.engine';"
             "assert build_vos_model.__module__=='aot_benchmark_b200.model';"
-            "assert A.__file__.startswith('/root/reference'); print('OK')") % (
-                REPO, os.path.join(REPO, "aot_benchmark_b200", "overlay"))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+            "assert E.build_engine is build_engine and E.build_vos_model is build_vos_model;"
+            "assert A.__file__.startswith(%r); print('OK')") % (
+                REPO, os.path.join(REPO, "aot_benchmark_b200", "overlay"), ref, ref)
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=str(tmp_path))
     assert "OK" in r.stdout, r.stderr[-1500:]
 
 
@@ -121,7 +132,7 @@ def test_kernel_register_budgets_fit_their_block_sizes():
     with 'too many resources requested' -- catch that here, without a GPU, from the cubin resource usage."""
     import re
     from aot_benchmark_b200 import _lib
-    r = subprocess.run(["cuobjdump", "-res-usage", _lib.LIB_PATH], capture_output=True, text=True)
+    r = _cuobjdump("-res-usage", _lib.LIB_PATH)
     if r.returncode != 0:
         pytest.skip("cuobjdump unavailable")
     blocks = {"lt_attn_tc_kernel": 576, "lt_attn_tc3_kernel": 576, "gp_attn_tc_kernel": 608, "conv_tc_kernel": 320, "local_attn_tile_kernel": 512,

@@ -2,7 +2,6 @@
 fixture produced by the REAL reference (oracle/gen_golden.py --only io), the product's size rule / palette / mask writer."""
 import io
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -65,8 +64,6 @@ def test_async_mask_writer_png_equals_reference(fx, tmp_path):
         assert a.getpalette() == b.getpalette()
 
 
-@pytest.mark.reference
-def test_palette_equals_the_reference_table():
-    sys.path.insert(0, os.environ.get("AOT_REFERENCE", "/root/reference"))
-    import utils.image as RI
-    assert IO.davis_palette() == RI._palette
+def test_palette_equals_the_reference_table(golden_dir):
+    from oracle.fixtures import load_reference_contract
+    assert IO.davis_palette() == load_reference_contract(golden_dir)["palette"]

@@ -156,28 +156,16 @@ def test_float64_oracle_close_to_float32():
     assert (outs[0] - outs[1]).abs().max().item() < 1e-4
 
 
-@pytest.mark.reference
-def test_state_dict_contract_against_reference():
-    """Our parameter trees expose exactly the reference's state_dict keys/shapes (SURVEY App. F)."""
-    import subprocess
-    import sys
-    code = r'''
-import sys
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, "%s")
-import networks.layers.transformer as T, networks.layers.attention as A
-T.MultiheadLocalAttentionV3 = A.MultiheadLocalAttentionV2
-from configs.default import DefaultEngineConfig
-from networks.models import build_vos_model as ref_build
-from aot_benchmark_b200 import build_vos_model, EngineConfig
-for m in ["aott", "r50_aotl", "deaott", "r50_deaotl", "swinb_aotl", "swinb_deaotl"]:
-    rc = DefaultEngineConfig("x", m); mc = EngineConfig("x", m)
-    a = {k: tuple(v.shape) for k, v in ref_build(rc.MODEL_VOS, rc).state_dict().items()}
-    b = {k: tuple(v.shape) for k, v in build_vos_model(mc.MODEL_VOS, mc).state_dict().items()}
-    assert a == b, m
-    for k, v in mc.__dict__.items():
-        if k not in ("EXP_NAME", "MODEL_NAME"):
-            assert getattr(rc, k) == v, (m, k)
-print("OK")
-''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
-    assert r.returncode == 0 and "OK" in r.stdout, r.stderr[-2000:]
+def test_state_dict_contract_against_reference(golden_dir):
+    """Our parameter trees expose exactly the reference's state_dict keys/shapes (SURVEY App. F), and every config value we
+    mirror equals the reference's (both recorded from the reference in tests/golden/reference_contract.json.gz)."""
+    from aot_benchmark_b200 import EngineConfig, build_vos_model
+    from oracle.fixtures import load_reference_contract
+    ref = load_reference_contract(golden_dir)["models"]
+    for m in ["aott", "r50_aotl", "deaott", "r50_deaotl", "swinb_aotl", "swinb_deaotl"]:
+        mc = EngineConfig("x", m)
+        b = {k: list(v.shape) for k, v in build_vos_model(mc.MODEL_VOS, mc).state_dict().items()}
+        assert ref[m]["state_dict"] == b, m
+        for k, v in mc.__dict__.items():
+            if k not in ("EXP_NAME", "MODEL_NAME"):
+                assert ref[m]["config"].get(k) == repr(v), (m, k)
